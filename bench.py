@@ -1,7 +1,7 @@
 #!/usr/bin/env python
 """bench.py -- the driver's benchmark contract for the PeRF per-ray hot path on B200.
 
-    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl ours|reference]
+    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl ours|reference] [--dump-outputs DIR]
 
 A "step" is one pass of the hot path over one synthetic batch: rendering ONE 1024x2048
 equirectangular panorama at 128 samples/ray (BASELINE.json configs[1]/[2] field: L=16 hash
@@ -17,6 +17,11 @@ JSON keys beyond the base contract:
   cpu_baseline  the oracle's plain-C / OpenMP port (oracle/cpath.c) on all host threads on a bounded
                 sample of the same rays; the PyTorch port (oracle/render.py) is reported beside it.
   e2e           same metric through the public API with a host pose in and host images out.
+
+--dump-outputs DIR writes what the last timed step rendered -- the whole panorama as a caller of
+render_pano receives it -- to DIR/rgb.npy [H,W,3], DIR/distance.npy [H,W,1] and DIR/opacities.npy
+[H,W,1], float32 (42 MB in all).  The field and the pose are seeded, so two builds run with the same
+arguments can be compared output for output.
 """
 from __future__ import annotations
 
@@ -30,6 +35,7 @@ import time
 
 ROOT = os.path.dirname(os.path.abspath(__file__))
 sys.path.insert(0, ROOT)
+sys.dont_write_bytecode = True                    # the benchmark leaves the source tree as it found it
 
 H, W, S = 1024, 2048, 128
 ALG_BYTES_PER_SAMPLE = 16 * 8 * 2 * 2 * 2        # levels x corners x features x sizeof(fp16) x fields
@@ -559,6 +565,8 @@ def run_ours(args, rank, world, local_rank):
     barrier()
     launches = ops.launch_count() - launches0
     total_ms = sum(e0.elapsed_time(e1) for e0, e1 in evs)
+    # the last timed step's panorama, before the end-to-end loop below renders into the same buffers
+    dumped = gather_panorama(out, rows_per, world) if args.dump_outputs else None
 
     # ---- end to end through the public API: host pose in, host images out, every step
     barrier()
@@ -583,6 +591,8 @@ def run_ours(args, rank, world, local_rank):
     total_ms, e2e_ms = (float(v) for v in t.tolist())
     if rank != 0:
         return
+    if dumped is not None:
+        write_outputs(args.dump_outputs, dumped)
     ms_per_step = total_ms / args.steps
     samples = H * W * S
     value = samples / (ms_per_step / 1e3) / 1e6
@@ -646,6 +656,31 @@ def run_ours(args, rank, world, local_rank):
     emit(line)
 
 
+def gather_panorama(out, rows_per, world):
+    """rgb / distance / opacities row tiles of every rank -> {name: [H, W, C] float32 on the host} on rank 0
+    (None elsewhere).  Tiles are padded to `rows_per` rows for the gather and cropped to H after it."""
+    import torch
+    import torch.distributed as dist
+    tile = torch.cat(out, -1)
+    if world > 1:
+        send = torch.zeros(rows_per, W, tile.shape[-1], dtype=tile.dtype, device=tile.device)
+        send[:tile.shape[0]] = tile
+        recv = [torch.empty_like(send) for _ in range(world)] if dist.get_rank() == 0 else None
+        dist.gather(send, recv, dst=0)
+        if recv is None:
+            return None
+        tile = torch.cat(recv)[:H]
+    tile = tile.cpu()
+    return {"rgb": tile[..., 0:3], "distance": tile[..., 3:4], "opacities": tile[..., 4:5]}
+
+
+def write_outputs(dirname, arrays):
+    import numpy as np
+    os.makedirs(dirname, exist_ok=True)
+    for name, t in arrays.items():
+        np.save(os.path.join(dirname, f"{name}.npy"), np.ascontiguousarray(t.numpy(), dtype=np.float32))
+
+
 _REAL_STDOUT = None
 
 
@@ -673,7 +708,12 @@ def main():
     ap.add_argument("--warmup", type=int, default=3)
     ap.add_argument("--impl", default="ours", choices=["ours", "reference"])
     ap.add_argument("--no-train", action="store_true", help="skip the secondary training-step measurement")
+    ap.add_argument("--dump-outputs", metavar="DIR", help="write the last timed step's rgb / distance / opacities to DIR/<name>.npy")
     args = ap.parse_args()
+    if args.steps < 1 or args.warmup < 0:
+        ap.error("--steps must be at least 1 and --warmup at least 0")
+    if args.dump_outputs and args.impl != "ours":
+        ap.error("--dump-outputs applies to --impl ours")
     rank, world, local_rank = int(os.environ.get("RANK", 0)), int(os.environ.get("WORLD_SIZE", 1)), int(os.environ.get("LOCAL_RANK", 0))
     if args.impl == "reference":
         run_reference(args, rank, world)

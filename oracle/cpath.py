@@ -9,6 +9,7 @@ import ctypes as C
 import hashlib
 import os
 import subprocess
+import tempfile
 
 import numpy as np
 import torch
@@ -26,10 +27,21 @@ def _cpu_tag() -> str:
 
 
 def build() -> str:
-    out_dir = os.path.join(HERE, "_build")
-    os.makedirs(out_dir, exist_ok=True)
+    """Up-to-date object under oracle/_build/, compiled there when the tree is writable, else in a temporary directory."""
     src = os.path.join(HERE, "cpath.c")
-    out = os.path.join(out_dir, f"liboracle_c_{_cpu_tag()}.so")
+    name = f"liboracle_c_{_cpu_tag()}.so"
+    out_dir = os.path.join(HERE, "_build")
+    out = os.path.join(out_dir, name)
+    if os.path.exists(out) and os.path.getmtime(src) <= os.path.getmtime(out):
+        return out
+    try:
+        os.makedirs(out_dir, exist_ok=True)
+    except OSError:
+        pass
+    if not os.access(out_dir, os.W_OK):
+        out_dir = os.path.join(tempfile.gettempdir(), f"perf_b200_oracle_{os.getuid()}")
+        os.makedirs(out_dir, exist_ok=True)
+        out = os.path.join(out_dir, name)
     if not os.path.exists(out) or os.path.getmtime(src) > os.path.getmtime(out):
         tmp = f"{out}.{os.getpid()}.tmp"
         cmd = ["gcc", "-O3", "-march=native", "-fopenmp", "-shared", "-fPIC", "-o", tmp, src, "-lm"]

@@ -1,7 +1,7 @@
-"""Generate the golden fixtures in this directory.  Run HERE (the build container), never
-on the GPU box: it imports the reference, which only exists at /root/reference.
+"""Generate the golden fixtures in this directory from a checkout of the original PeRF project
+(the reference): it imports the reference's own files, so the tests never need that checkout.
 
-    python tests/golden/make_golden.py
+    python tests/golden/make_golden.py <path to the PeRF checkout>
 
 What is the reference's own code and what is restated:
 
@@ -14,6 +14,14 @@ What is the reference's own code and what is restated:
 * ``render.npz``   -- `modules/scene/nerf_renderer.py` ``NeRFOCCRenderer.render`` imported
   unmodified, on CPU stand-ins for ``nerfacc`` (``oracle.composite``) and an estimator
   whose ``sampling`` returns the fixed-S intervals of ``oracle.sampler``.
+
+* ``reference_host.npz`` / ``reference_api.json`` -- the host-side files the CPU tests compare
+  with: `modules/pose_sampler/`, `modules/dataset/sup_info.py` (``kornia`` bound to the
+  restatements in perf_b200/sup_info.py), ``NeRFScene.update_lr`` / ``gen_occ_grid`` /
+  ``to_bounded_rays``, the tinycudann constructor calls of `modules/fields/ngp_nerf.py` and
+  the names the reference imports from its three plugin packages, all run on the
+  perf_b200 shims; plus the parsed YAML of `configs/nerf.yaml` and the defaults it selects.
+* ``sup_info.npz`` -- a summary of the ``SupInfoPool`` of tests/test_sup_info.py.
 
 So the glue (aabb normalise, selector, trunc_exp, sample-position rule, weights.detach,
 background rules, dtype promotions) is pinned by the reference itself; the third-party
@@ -30,7 +38,7 @@ import torch
 
 HERE = os.path.dirname(os.path.abspath(__file__))
 ROOT = os.path.dirname(os.path.dirname(HERE))
-REF = "/root/reference"
+REF = None                                   # the PeRF checkout, from the command line
 sys.path.insert(0, ROOT)
 
 import oracle  # noqa: E402
@@ -174,8 +182,176 @@ def make_field_and_render():
     np.savez_compressed(os.path.join(HERE, "render.npz"), **out_r)
 
 
+def install_host_stand_ins():
+    """The perf_b200 plugin shims, ``kornia`` bound to perf_b200's restatements, and empty modules for the
+    reference's third-party imports that the host-side files do not use on these paths."""
+    from perf_b200 import shims
+    from perf_b200 import sup_info as S
+    for m in [k for k in sys.modules if k.split(".")[0] in ("modules", "utils", "tinycudann", "nerfacc")]:
+        del sys.modules[m]
+    shims.install()
+    kornia = types.ModuleType("kornia"); filters = types.ModuleType("kornia.filters"); morph = types.ModuleType("kornia.morphology")
+    filters.laplacian = lambda x, kernel_size: S.laplacian3(x) if kernel_size == 3 else None
+    morph.erosion = lambda x, kernel: S.erosion(x, kernel)
+    morph.dilation = lambda x, kernel: S.dilation(x, kernel)
+    kornia.filters, kornia.morphology = filters, morph
+    trimesh = types.ModuleType("trimesh"); creation = types.ModuleType("trimesh.creation")
+    creation.icosphere = lambda *a, **k: None
+    trimesh.creation = creation
+    icecream = types.ModuleType("icecream"); icecream.ic = print
+    sys.modules.update({"kornia": kornia, "kornia.filters": filters, "kornia.morphology": morph, "trimesh": trimesh,
+                        "trimesh.creation": creation, "icecream": icecream})
+    sys.modules.setdefault("imageio", types.ModuleType("imageio"))
+    if REF not in sys.path:
+        sys.path.insert(1, REF)
+
+
+def shim_names_used():
+    """{plugin package: sorted names} the reference's files import from it or read off it (``tcnn.X``)."""
+    import ast
+    out = {}
+    for dirpath, _, files in os.walk(os.path.join(REF, "modules")):
+        for f in files:
+            if not f.endswith(".py"):
+                continue
+            tree = ast.parse(open(os.path.join(dirpath, f)).read())
+            aliases = {}
+            for node in ast.walk(tree):
+                if isinstance(node, ast.ImportFrom) and node.module and node.module.split(".")[0] in ("nerfacc", "torch_efficient_distloss", "tinycudann"):
+                    out.setdefault(node.module, set()).update(a.name for a in node.names)
+                elif isinstance(node, ast.Import):
+                    for a in node.names:
+                        if a.name == "tinycudann":
+                            aliases[a.asname or a.name] = a.name
+            for node in ast.walk(tree):
+                if isinstance(node, ast.Attribute) and isinstance(node.value, ast.Name) and node.value.id in aliases:
+                    out.setdefault(aliases[node.value.id], set()).add(node.attr)
+    return {k: sorted(v) for k, v in sorted(out.items())}
+
+
+def make_reference_host():
+    import hashlib
+    import json
+    import yaml
+    from types import SimpleNamespace
+    sys.path.insert(1, os.path.dirname(HERE))                        # tests/: the inputs the tests build
+    import test_runner_host
+    import test_sup_info as T
+    install_host_stand_ins()
+    arrays, api = {}, {}
+
+    # -- tinycudann constructor calls of ngp_nerf.py, on the shim
+    import tinycudann
+    calls, shim_cls = [], tinycudann.NetworkWithInputEncoding
+
+    class Recording(shim_cls):
+        def __init__(self, *a, **k):
+            kw = dict(zip(("n_input_dims", "n_output_dims", "encoding_config", "network_config"), a), **k)
+            calls.append(kw)
+            super().__init__(**kw)
+    tinycudann.NetworkWithInputEncoding = Recording
+    from modules.fields import ngp_nerf
+    f = ngp_nerf.NGPNeRF(aabb=[-1.0, -1.0, -1.0, 1.0, 1.0, 1.0])
+    api["tcnn_calls"] = {"NGPNeRF": calls[:]}
+    api["nerf_state_dict"] = {k: {"shape": list(v.shape), "dtype": str(v.dtype)} for k, v in f.state_dict().items()}
+    del calls[:]
+    f.reset_geo()
+    api["tcnn_calls"]["NGPNeRF.reset_geo"] = calls[:]
+    del calls[:]
+    try:
+        ngp_nerf.NGPDensityField(aabb=[-1.0, -1.0, -1.0, 1.0, 1.0, 1.0])
+    except RuntimeError:                                             # the shim refuses the proposal field's 10-wide input
+        pass
+    api["tcnn_calls"]["NGPDensityField"] = calls[:]
+    tinycudann.NetworkWithInputEncoding = shim_cls
+    api["shim_names"] = shim_names_used()
+    from modules.scene import nerf_renderer
+    from modules.scene import nerf as nerf_scene
+    api["renderer_state_dict_keys"] = sorted(nerf_renderer.NeRFOCCRenderer(max_radius=2, bg_color="rand_noise").state_dict())
+
+    # -- configs/nerf.yaml and the defaults it selects, parsed; the LR schedule of NeRFScene.update_lr on it
+    root = yaml.safe_load(open(os.path.join(REF, "configs", "nerf.yaml")))
+    api["configs"] = {"nerf.yaml": root}
+    for item in root["defaults"]:
+        for group, choice in (item.items() if isinstance(item, dict) else ()):
+            api["configs"][f"{group}/{choice}.yaml"] = yaml.safe_load(open(os.path.join(REF, "configs", group, f"{choice}.yaml")))
+    oc = SimpleNamespace(**{k: float(v) for k, v in root["scene"]["train_conf"]["geo_optimizer"].items()})
+    opt = SimpleNamespace(param_groups=[{"lr": 0.0}])
+    progress, lrs = [i / 3000 for i in range(0, 3000, 37)], []
+    for p in progress:
+        nerf_scene.NeRFScene.update_lr(None, opt, oc, p)
+        lrs.append(opt.param_groups[0]["lr"])
+    api["lr_schedule"] = {"progress": progress, "geo_optimizer_lr": lrs}
+
+    # -- SupInfoPool.gen_occ_grid and to_bounded_rays (inputs of tests/test_shims_reference_import.py)
+    from modules.dataset import sup_info as ref
+    from utils.camera_utils import Rays as RefRays
+    g = torch.Generator().manual_seed(0)
+    n = 5000
+    o = (torch.rand(n, 3, generator=g) - .5) * .2
+    d = torch.nn.functional.normalize(torch.randn(n, 3, generator=g), dim=-1)
+    dist = torch.rand(n, 1, generator=g) * .8 + .05
+    grid, pts = ref.SupInfoPool.gen_occ_grid(SimpleNamespace(all_sup_rays=RefRays(o, d), all_sup_distances=dist), res=32)
+    arrays["occ32_grid"], arrays["occ32_pts"] = grid.numpy(), pts.numpy()
+    br = nerf_scene.NeRFScene.to_bounded_rays(None, RefRays(o, d))
+    arrays["bounded_near"], arrays["bounded_far"] = br.near.numpy(), br.far.numpy()
+
+    # -- pose samplers on the distance map of tests/test_runner_host.py (the reference hard-codes .cuda())
+    saved_cuda = torch.Tensor.cuda
+    torch.Tensor.cuda = lambda self, *a, **k: self
+    try:
+        from modules.pose_sampler import circle_pose_sampler, dense_travel_pose_sampler
+        circle = circle_pose_sampler.CirclePoseSampler(test_runner_host._distance_map(), traverse_ratios=[0.2, 0.4, 0.6],
+                                                       n_anchors_per_ratio=[8, 8, 8])
+        for name in ("plane_pts_raw", "plane_pts_filter", "plane_pts_smooth", "anchor_pts", "traverse_pts", "traverse_normals"):
+            arrays[f"circle_{name}"] = getattr(circle, name).numpy()
+        arrays["circle_n_anchors"] = np.array(circle.n_anchors)
+        arrays["circle_sample_pose_5"] = circle.sample_pose(5).numpy()
+        np.random.seed(0)
+        arrays["dense_sample_poses"] = dense_travel_pose_sampler.DenseTravelPoseSampler(circle, n_dense_poses=12).sample_poses.numpy()
+    finally:
+        torch.Tensor.cuda = saved_cuda
+
+    # -- SupInfoPool of tests/test_sup_info.py
+    scene = T._scene()
+    pool = T._pool(ref.SupInfoPool, *scene)
+    for i, info in enumerate(pool.sup_infos):
+        for name in T.POOL_INFO_FIELDS:
+            arrays[f"pool{i}_{name}"] = getattr(info, name).numpy()
+    arrays["pool_all_sup_colors"], arrays["pool_all_sup_dirs"] = pool.all_sup_colors.numpy(), pool.all_sup_rays.d.numpy()
+    arrays["pool_all_sup_distances"], arrays["pool_all_sup_normals"] = pool.all_sup_distances.numpy(), pool.all_sup_normals.numpy()
+    rays, distances = T._probe(pool, 40, 80, scene[4])
+    arrays["pool_geo_check"] = pool.geo_check(ref.Rays(rays.o, rays.d), distances).numpy()
+    grid, pts = pool.gen_occ_grid(32)
+    arrays["pool_occ32_grid"], arrays["pool_occ32_pts"] = grid.numpy(), pts.numpy()
+    torch.manual_seed(5)
+    r, c, dd, nn = pool.rand_ray_color_data(64)
+    arrays.update(pool_draw64_dirs=r.d.numpy(), pool_draw64_colors=c.numpy(), pool_draw64_distances=dd.numpy(), pool_draw64_normals=nn.numpy())
+    for mode in ("only_first", "only_last"):
+        torch.manual_seed(6)
+        r, c, _, _ = pool.rand_ray_color_data(32, rand_mode=mode)
+        arrays[f"pool_draw32_{mode}_dirs"], arrays[f"pool_draw32_{mode}_colors"] = r.d.numpy(), c.numpy()
+    sd = pool.state_dict()
+    api["sup_pool_state_dict_keys"] = {"pool": sorted(sd), "sup_info_0": sorted(sd["sup_info_0"])}
+    np.savez_compressed(os.path.join(HERE, "sup_info.npz"), **T._golden_payload(T._pool(ref.SupInfoPool, *scene), scene))
+
+    # the large float arrays of the pool are compared bit for bit: their digests keep the fixture small
+    api["pool_sha256"] = {}
+    for k in [k for k in arrays if k.startswith("pool") and arrays[k].dtype.kind == "f" and arrays[k].size >= 4096]:
+        a = np.ascontiguousarray(arrays.pop(k))
+        api["pool_sha256"][k] = {"shape": list(a.shape), "dtype": str(a.dtype), "sha256": hashlib.sha256(a.tobytes()).hexdigest()}
+    np.savez_compressed(os.path.join(HERE, "reference_host.npz"), **arrays)
+    with open(os.path.join(HERE, "reference_api.json"), "w") as fh:
+        json.dump(api, fh, indent=1, sort_keys=True)
+        fh.write("\n")
+
+
 if __name__ == "__main__":
+    if len(sys.argv) != 2:
+        sys.exit(__doc__)
+    REF = os.path.abspath(sys.argv[1])
     make_raygen()
     make_field_and_render()
-    for f in ("raygen.npz", "field.npz", "render.npz"):
+    make_reference_host()
+    for f in ("raygen.npz", "field.npz", "render.npz", "sup_info.npz", "reference_host.npz", "reference_api.json"):
         print(f, os.path.getsize(os.path.join(HERE, f)))

@@ -1,8 +1,8 @@
-"""CPU tests of the host-side callers of the path: pose samplers (against the reference's own files),
-dataset file formats, config -> runner plumbing that does not need a GPU."""
+"""CPU tests of the host-side callers of the path: pose samplers (against what the reference's own files
+computed on the same distance map, tests/golden/reference_host.npz), dataset file formats, config -> runner
+plumbing that does not need a GPU."""
+import json
 import os
-import sys
-import types
 
 import numpy as np
 import pytest
@@ -11,7 +11,7 @@ import torch
 from perf_b200 import pose_sampler as P
 from perf_b200.synthetic import box_room_distance, smooth_rgb
 
-REF = "/root/reference"
+GOLDEN = os.path.join(os.path.dirname(os.path.abspath(__file__)), "golden")
 
 
 def _distance_map(h=64, w=128):
@@ -20,47 +20,23 @@ def _distance_map(h=64, w=128):
     return d / (d.max() * 1.05)
 
 
-@pytest.fixture(scope="module")
-def reference_pose_samplers():
-    if not os.path.isdir(REF):
-        pytest.skip("reference checkout not present on this machine")
-    saved_path, saved_mods = list(sys.path), dict(sys.modules)
-    trimesh = types.ModuleType("trimesh"); creation = types.ModuleType("trimesh.creation")
-    creation.icosphere = lambda *a, **k: None
-    trimesh.creation = creation
-    icecream = types.ModuleType("icecream"); icecream.ic = print
-    for name, m in {"trimesh": trimesh, "trimesh.creation": creation, "icecream": icecream}.items():
-        sys.modules.setdefault(name, m)
-    sys.path.insert(1, REF)
-    saved_cuda = torch.Tensor.cuda
-    torch.Tensor.cuda = lambda self, *a, **k: self               # the reference hard-codes .cuda(); no GPU here
-    try:
-        from modules.pose_sampler import circle_pose_sampler, dense_travel_pose_sampler
-        yield circle_pose_sampler, dense_travel_pose_sampler
-    finally:
-        torch.Tensor.cuda = saved_cuda
-        sys.path[:] = saved_path
-        for k in [k for k in sys.modules if k not in saved_mods]:
-            del sys.modules[k]
-
-
-def test_pose_samplers_match_reference_files(reference_pose_samplers):
-    ref_circle, ref_dense = reference_pose_samplers
+def test_pose_samplers_match_reference_files():
+    ref = np.load(os.path.join(GOLDEN, "reference_host.npz"))
     d = _distance_map()
     kw = dict(traverse_ratios=[0.2, 0.4, 0.6], n_anchors_per_ratio=[8, 8, 8])       # configs/nerf.yaml:16-18
-    want, got = ref_circle.CirclePoseSampler(d.clone(), **kw), P.CirclePoseSampler(d.clone(), **kw)
-    assert want.n_anchors == got.n_anchors == 24 and got.n_poses == 24
+    got = P.CirclePoseSampler(d.clone(), **kw)
+    assert int(ref["circle_n_anchors"]) == got.n_anchors == 24 and got.n_poses == 24
     for name in ("plane_pts_raw", "plane_pts_filter", "plane_pts_smooth", "anchor_pts", "traverse_pts", "traverse_normals"):
-        assert torch.equal(getattr(want, name), getattr(got, name)), name
-    assert torch.equal(want.sample_pose(5), got.sample_pose(5))
+        want = torch.from_numpy(ref[f"circle_{name}"])
+        assert getattr(got, name).dtype == want.dtype and torch.equal(getattr(got, name), want), name
+    assert torch.equal(torch.from_numpy(ref["circle_sample_pose_5"]), got.sample_pose(5))
     # anchors stay inside the room: closer to the origin than the wall in their direction
     assert got.anchor_pts.norm(dim=-1).max() < 0.7 * float(d.max())
     np.random.seed(0)
-    dense_want = ref_dense.DenseTravelPoseSampler(want, n_dense_poses=12)
-    np.random.seed(0)
     dense_got = P.DenseTravelPoseSampler(got, n_dense_poses=12)
-    assert dense_want.n_poses == dense_got.n_poses and 10 <= dense_got.n_poses <= 14
-    assert torch.equal(dense_want.sample_poses, dense_got.sample_poses)
+    dense_want = torch.from_numpy(ref["dense_sample_poses"])
+    assert len(dense_want) == dense_got.n_poses and 10 <= dense_got.n_poses <= 14
+    assert torch.equal(dense_want, dense_got.sample_poses)
     rot = dense_got.sample_poses[:, :3, :3]
     assert torch.allclose(rot @ rot.transpose(1, 2), torch.eye(3).expand_as(rot), atol=1e-5)
 
@@ -98,9 +74,9 @@ def test_wild_dataset_formats(tmp_path):
 def test_runner_config_plumbing_without_gpu(tmp_path):
     """The reference's YAML drives the runner unchanged; without a CUDA device constructing the scene fails loudly."""
     from perf_b200.config import load_config
-    if not os.path.isdir(REF):
-        pytest.skip("reference checkout not present on this machine")
-    conf = load_config(os.path.join(REF, "configs"), "nerf", ["exp_name=t", "scene.train_conf.raw_phase_iter_geo=10"])
+    from test_shims_reference_import import write_reference_configs
+    config_dir = write_reference_configs(tmp_path, json.load(open(os.path.join(GOLDEN, "reference_api.json"))))
+    conf = load_config(config_dir, "nerf", ["exp_name=t", "scene.train_conf.raw_phase_iter_geo=10"])
     assert conf.scene.estimator_type == "occ" and conf.scene.train_conf.raw_phase_iter_geo == 10
     assert conf.pose_sampler.n_anchors_per_ratio == [8, 8, 8] and conf.device.base_exp_dir == "."
     assert conf.dataset.image_resize == [2048, 1024]

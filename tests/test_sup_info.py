@@ -2,14 +2,14 @@
 
 * the three kornia 0.7.0 functions restated there are pinned against OpenCV (an independent
   implementation of the same filters);
-* ``PanoSupInfo`` / ``SupInfoPool`` are compared with the reference's OWN `modules/dataset/sup_info.py`,
-  imported unmodified with ``kornia`` bound to those restatements (build container only);
-* a committed fixture (``tests/golden/sup_info.npz``, minted by that same import) travels to machines
-  without /root/reference.
+* ``PanoSupInfo`` / ``SupInfoPool`` are compared with what the reference's OWN `modules/dataset/sup_info.py`,
+  imported unmodified with ``kornia`` bound to those restatements, computed on the same inputs: the
+  fixtures ``tests/golden/reference_host.npz`` / ``reference_api.json`` and the summary
+  ``tests/golden/sup_info.npz`` (all minted by tests/golden/make_golden.py).
 """
+import hashlib
+import json
 import os
-import sys
-import types
 
 import cv2
 import numpy as np
@@ -19,8 +19,11 @@ import torch
 from perf_b200 import sup_info as S
 from perf_b200.synthetic import box_room_distance, smooth_rgb
 
-REF = "/root/reference"
 GOLDEN = os.path.join(os.path.dirname(__file__), "golden", "sup_info.npz")
+REFERENCE_HOST = os.path.join(os.path.dirname(__file__), "golden", "reference_host.npz")
+REFERENCE_API = os.path.join(os.path.dirname(__file__), "golden", "reference_api.json")
+POOL_INFO_FIELDS = ("mask_raw", "mask", "color_map", "distance_map", "normal_map", "sup_colors", "sup_distances",
+                    "sup_normals", "sup_dirs", "sup_positions", "pose")
 
 
 # ------------------------------------------------------------------ kornia restatements vs OpenCV
@@ -84,69 +87,53 @@ def _probe(pool, h, w, pose):
     return rays, distances
 
 
-@pytest.fixture(scope="module")
-def reference_sup_info():
-    if not os.path.isdir(REF):
-        pytest.skip("reference checkout not present on this machine")
-    saved_path, saved_mods = list(sys.path), dict(sys.modules)
-    kornia = types.ModuleType("kornia"); filters = types.ModuleType("kornia.filters"); morph = types.ModuleType("kornia.morphology")
-    filters.laplacian = lambda x, kernel_size: S.laplacian3(x) if kernel_size == 3 else None
-    morph.erosion = lambda x, kernel: S.erosion(x, kernel)
-    morph.dilation = lambda x, kernel: S.dilation(x, kernel)
-    kornia.filters, kornia.morphology = filters, morph
-    trimesh = types.ModuleType("trimesh"); creation = types.ModuleType("trimesh.creation")
-    creation.icosphere = lambda *a, **k: None
-    trimesh.creation = creation
-    icecream = types.ModuleType("icecream"); icecream.ic = print
-    imageio = types.ModuleType("imageio")
-    for name, m in {"kornia": kornia, "kornia.filters": filters, "kornia.morphology": morph, "trimesh": trimesh,
-                    "trimesh.creation": creation, "icecream": icecream}.items():
-        sys.modules[name] = m
-    sys.modules.setdefault("imageio", imageio)
-    sys.path.insert(1, REF)
-    from modules.dataset import sup_info as ref
-    yield ref
-    sys.path[:] = saved_path
-    for k in [k for k in sys.modules if k not in saved_mods]:
-        del sys.modules[k]
-    for k, v in saved_mods.items():
-        sys.modules[k] = v
+def test_pool_matches_reference_file():
+    arrays, api = np.load(REFERENCE_HOST), json.load(open(REFERENCE_API))
 
-
-def test_pool_matches_reference_file(reference_sup_info):
-    ref = reference_sup_info
+    def _same(got: torch.Tensor, key: str, name: str):
+        """Bit-identical to the reference's array (stored, or as shape, dtype and SHA-256 of its bytes)."""
+        if key in arrays.files:
+            want = torch.from_numpy(arrays[key])
+            assert got.dtype == want.dtype and torch.equal(got, want), name
+        else:
+            a = np.ascontiguousarray(got.numpy())
+            assert api["pool_sha256"][key] == {"shape": list(a.shape), "dtype": str(a.dtype),
+                                               "sha256": hashlib.sha256(a.tobytes()).hexdigest()}, name
     scene = _scene()
-    want, got = _pool(ref.SupInfoPool, *scene), _pool(lambda: S.SupInfoPool(locality_sort=False), *scene)
-    for a, b in zip(want.sup_infos, got.sup_infos):
-        for name in ("mask_raw", "mask", "color_map", "distance_map", "normal_map", "sup_colors", "sup_distances",
-                     "sup_normals", "sup_dirs", "sup_positions", "pose"):
-            assert torch.equal(getattr(a, name), getattr(b, name)), name
+    got = _pool(lambda: S.SupInfoPool(locality_sort=False), *scene)
+    for i, b in enumerate(got.sup_infos):
+        for name in POOL_INFO_FIELDS:
+            _same(getattr(b, name), f"pool{i}_{name}", f"{name} of panorama {i}")
     assert 0.3 < got.sup_infos[0].mask.float().mean() < 0.95          # the masks do remove something
-    assert torch.equal(want.all_sup_colors, got.all_sup_colors) and torch.equal(want.all_sup_rays.d, got.all_sup_rays.d)
-    assert torch.equal(want.all_sup_distances, got.all_sup_distances) and torch.equal(want.all_sup_normals, got.all_sup_normals)
+    _same(got.all_sup_colors, "pool_all_sup_colors", "all_sup_colors")
+    _same(got.all_sup_rays.d, "pool_all_sup_dirs", "all_sup_rays.d")
+    _same(got.all_sup_distances, "pool_all_sup_distances", "all_sup_distances")
+    _same(got.all_sup_normals, "pool_all_sup_normals", "all_sup_normals")
     # geo_check on a novel view
     rays, distances = _probe(got, 40, 80, scene[4])
-    m_want = want.geo_check(ref.Rays(rays.o, rays.d), distances)
     m_got = got.geo_check(rays, distances)
-    assert torch.equal(m_want, m_got) and 0.02 < m_got.mean() < 0.98
+    _same(m_got, "pool_geo_check", "geo_check")
+    assert 0.02 < m_got.mean() < 0.98
     # occupancy pre-grid
-    g_want, p_want = want.gen_occ_grid(32)
     g_got, p_got = got.gen_occ_grid(32)
-    assert torch.equal(g_want, g_got) and torch.equal(p_want, p_got)
+    _same(g_got, "pool_occ32_grid", "gen_occ_grid")
+    _same(p_got, "pool_occ32_pts", "gen_occ_grid points")
     # batch sampler: the same draw from the same generator state
-    torch.manual_seed(5)
-    r_w, c_w, d_w, n_w = want.rand_ray_color_data(64)
     got.use_default_generator = True
     torch.manual_seed(5)
     r_g, c_g, d_g, n_g = got.rand_ray_color_data(64)
-    assert torch.equal(r_w.d, r_g.d) and torch.equal(c_w, c_g) and torch.equal(d_w, d_g) and torch.equal(n_w, n_g)
+    _same(r_g.d, "pool_draw64_dirs", "draw dirs")
+    _same(c_g, "pool_draw64_colors", "draw colors")
+    _same(d_g, "pool_draw64_distances", "draw distances")
+    _same(n_g, "pool_draw64_normals", "draw normals")
     for mode in ("only_first", "only_last"):
-        torch.manual_seed(6); a = want.rand_ray_color_data(32, rand_mode=mode)
         torch.manual_seed(6); b = got.rand_ray_color_data(32, rand_mode=mode)
-        assert torch.equal(a[1], b[1]) and torch.equal(a[0].d, b[0].d)
+        _same(b[1], f"pool_draw32_{mode}_colors", mode)
+        _same(b[0].d, f"pool_draw32_{mode}_dirs", mode)
     # checkpoint keys (incl. the reference's unformatted height / width keys)
-    assert set(want.state_dict()) == set(got.state_dict())
-    assert set(want.state_dict()["sup_info_0"]) == set(got.state_dict()["sup_info_0"])
+    keys = api["sup_pool_state_dict_keys"]
+    assert sorted(got.state_dict()) == keys["pool"]
+    assert sorted(got.state_dict()["sup_info_0"]) == keys["sup_info_0"]
 
 
 def _golden_payload(pool, scene):
@@ -159,7 +146,7 @@ def _golden_payload(pool, scene):
 
 
 def test_pool_matches_golden_fixture():
-    """The fixture was written from the reference's own file (``python tests/test_sup_info.py``)."""
+    """The fixture was written from the reference's own file (tests/golden/make_golden.py)."""
     scene = _scene()
     got = _golden_payload(_pool(lambda: S.SupInfoPool(locality_sort=False), *scene), scene)
     want = np.load(GOLDEN)
@@ -189,14 +176,6 @@ def test_locality_sort_keeps_the_multiset_and_checkpoint_roundtrip():
     assert vis[info.mask[..., 0]].mean() > 0.9
     far_vis = sorted_.pano_visibility_mask(rays, info.distance_map * 1.5)          # behind the surface: hidden
     assert far_vis.mean() < 0.2
-
-
-if __name__ == "__main__":        # mint tests/golden/sup_info.npz from the reference's own file
-    gen = reference_sup_info.__wrapped__()
-    ref = next(gen)
-    sc = _scene()
-    np.savez_compressed(GOLDEN, **_golden_payload(_pool(ref.SupInfoPool, *sc), sc))
-    print("wrote", GOLDEN)
 
 
 def test_factor_downsampling_is_opencv_inter_area():
