@@ -207,6 +207,28 @@ int perf_render_packed(const perf_render_args* args, const float* d_rays_o, cons
 int perf_render_pano(const perf_render_args* args, const float* h_pose, int H, int W,
                      int row0, int rows, void* stream);
 
+/* ---- one-launch render with the occupancy-grid sampler (nerf_renderer.py:145-197 in eval mode) ----
+ * Each ray walks the grid itself (the intervals of perf_occ_count / perf_occ_write with no jitter, bit for bit),
+ * evaluates both fields at each interval it emits and composites it, and stops at its first interval whose exclusive
+ * transmittance exp(-sum_{j<i} sigma_j dt_j) is below early_stop_eps (nerfacc render_visibility_from_density with
+ * alpha_thre = 0).  Nothing per sample is written.  Of perf_render_args, n_samples / near / far / d_jitter / d_bg_noise
+ * are ignored; PERF_FLAG_SIMT_MLP and PERF_FLAG_GENERIC_ADDR are honoured, PERF_FLAG_TRAINING / _SCAN_KERNEL / _L0_SMEM
+ * return PERF_EUNSUPPORTED; eval-mode background rule. */
+typedef struct perf_occ_render_args {
+    const uint8_t* d_binaries;        /* [res0][res1][res2] bool/uint8, x slowest (OccGridEstimator.binaries[0])        */
+    int            res[3];
+    float          aabb[6];           /* the estimator's roi_aabb (independent of perf_render_args.aabb, the field's)    */
+    float          near, far, step;   /* PeRF: 0, 1.5, 5e-4 (nerf_renderer.py:149-151)                                 */
+    float          early_stop_eps;    /* PeRF: 1e-4 (nerfacc default); 0 = keep every interval; must be in [0, 1)       */
+    uint32_t*      d_n_samples;       /* [R] intervals composited per ray, or NULL                                     */
+} perf_occ_render_args;
+/* Explicit rays d_rays_o / d_rays_d [R,3] fp32 (args->image_width as for perf_render_rays). */
+int perf_render_rays_occ(const perf_render_args* args, const perf_occ_render_args* occ, const float* d_rays_o,
+                         const float* d_rays_d, uint64_t R, void* stream);
+/* Rows [row0,row0+rows) of an H x W equirect panorama, ray generation fused in (as perf_render_pano). */
+int perf_render_pano_occ(const perf_render_args* args, const perf_occ_render_args* occ, const float* h_pose,
+                         int H, int W, int row0, int rows, void* stream);
+
 /* ---- fused training step (fixed-S sampler): forward with saves, composite backward, grid scatter ----
  * All per-sample buffers are SAMPLE-MAJOR: row = k * R + ray (k = sample index along the ray), so
  * that a warp of neighbouring rays reads/writes contiguous rows.  Replaces, for one optimisation

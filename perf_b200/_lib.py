@@ -39,6 +39,11 @@ class RenderArgs(C.Structure):
                 ("d_jitter", vp), ("d_bg_noise", vp), ("d_rgb", vp), ("d_distance", vp), ("d_opacity", vp), ("image_width", u32)]
 
 
+class OccRenderArgs(C.Structure):
+    _fields_ = [("d_binaries", vp), ("res", i32 * 3), ("aabb", f32 * 6), ("near", f32), ("far", f32), ("step", f32),
+                ("early_stop_eps", f32), ("d_n_samples", vp)]
+
+
 P_u32 = C.POINTER(u32)
 PERF_MAX_SEGMENTS = 64
 
@@ -75,6 +80,8 @@ SIGNATURES = {
     "perf_render_rays": (i32, [P(RenderArgs), vp, vp, u64, vp]),
     "perf_render_packed": (i32, [P(RenderArgs), vp, vp, u64, vp, vp, vp, vp]),
     "perf_render_pano": (i32, [P(RenderArgs), P(f32), i32, i32, i32, i32, vp]),
+    "perf_render_rays_occ": (i32, [P(RenderArgs), P(OccRenderArgs), vp, vp, u64, vp]),
+    "perf_render_pano_occ": (i32, [P(RenderArgs), P(OccRenderArgs), P(f32), i32, i32, i32, i32, vp]),
     "perf_train_forward": (i32, [P(RenderArgs), vp, vp, u64, i32, P(TrainBuffers), vp]),
     "perf_train_backward_composite": (i32, [i32, u32, u32, f32, f32, u64, vp, vp, P(TrainBuffers), vp, vp, vp, vp, vp, vp, vp, vp]),
     "perf_hashgrid_bwd_rays": (i32, [P(GridCfg), P(f32), vp, vp, vp, u64, u32, f32, f32, vp, vp, vp]),

@@ -12,6 +12,7 @@
 //   gen_pano_rays                       utils/camera_utils.py:229-234
 // Arithmetic contract: oracle/render.py::render_rays(mixed=True).
 #include "mlp_tc.cuh"
+#include "occ_walk.cuh"
 
 namespace perf {
 
@@ -540,6 +541,52 @@ __global__ void __launch_bounds__(TILE, 4) render_kernel(const __grid_constant__
 }
 
 
+// The ray of thread `tid` in work tile `tile` of the ray-marching kernels: a PATCH_W x PATCH_H pixel patch of the panorama
+// window (PANO) or of a row-major image of explicit rays (patch), otherwise `rpt` consecutive explicit rays.  The origin and
+// direction are left as they are for a thread without a ray (valid == false).  render_march_kernel has the same selection
+// written inline: routed through this function, ptxas allocates its registers differently, and the benchmarked kernel's
+// code is kept as measured.
+template <bool PANO>
+__device__ __forceinline__ void march_tile_ray(const RenderArgs& a, uint64_t tile, bool patch, uint32_t tiles_x, int rows, uint32_t rpt, int tid,
+                                               uint64_t& ray, bool& valid, float& ox, float& oy, float& oz, float& dx, float& dy, float& dz)
+{
+    const int warp = tid >> 5, lane = tid & 31;
+    if constexpr (PANO) {
+        const int ty = (int)(tile / tiles_x), tx = (int)(tile % tiles_x);
+        const int prow = ty * PATCH_H + (warp / PATCH_WX) * PATCH_WH + lane / PATCH_WW;   // row inside the window
+        const int pcol = tx * PATCH_W + (warp % PATCH_WX) * PATCH_WW + lane % PATCH_WW;
+        valid = prow < rows && pcol < a.W;
+        ray = (uint64_t)prow * (uint64_t)a.W + (uint64_t)pcol;
+        if (valid) {
+            const float yy = linspace_val_r(a.row0 + prow, a.H), xx = linspace_val_r(pcol, a.W);
+            const float beta = -(yy - 0.5f) * 3.14159274101257324f;
+            const float alpha = -(xx - 0.5f) * 6.28318548202514648f;
+            float sa, ca, sb, cb;
+            sincosf(alpha, &sa, &ca); sincosf(beta, &sb, &cb);
+            const float cx = ca * cb, cy = sa * cb, cz = sb;
+            dx = a.pose_r[0] * cx + a.pose_r[1] * cy + a.pose_r[2] * cz;
+            dy = a.pose_r[3] * cx + a.pose_r[4] * cy + a.pose_r[5] * cz;
+            dz = a.pose_r[6] * cx + a.pose_r[7] * cy + a.pose_r[8] * cz;
+            ox = a.pose_t[0]; oy = a.pose_t[1]; oz = a.pose_t[2];
+        }
+    } else {
+        if (patch) {
+            const int ty = (int)(tile / tiles_x), tx = (int)(tile % tiles_x);
+            const int prow = ty * PATCH_H + (warp / PATCH_WX) * PATCH_WH + lane / PATCH_WW;
+            const int pcol = tx * PATCH_W + (warp % PATCH_WX) * PATCH_WW + lane % PATCH_WW;
+            valid = prow < rows && pcol < a.W;
+            ray = (uint64_t)prow * (uint64_t)a.W + (uint64_t)pcol;
+        } else {
+            ray = tile * rpt + (uint32_t)tid % rpt;
+            valid = ray < a.R;
+        }
+        if (valid) {
+            ox = a.rays_o[3 * ray]; oy = a.rays_o[3 * ray + 1]; oz = a.rays_o[3 * ray + 2];
+            dx = a.rays_d[3 * ray]; dy = a.rays_d[3 * ray + 1]; dz = a.rays_d[3 * ray + 2];
+        }
+    }
+}
+
 // ------------------------------------------------------------------------------------------------
 // render_march_kernel: thread = RAY, the 128 rows of an MMA tile are 128 neighbouring rays at the
 // same sample index k.  For a panorama a warp is an 8x4 pixel patch and a CTA a 16x8 patch, so the
@@ -768,6 +815,117 @@ __global__ void __launch_bounds__(TILE, L0SMEM ? 3 : 4) render_march_kernel(cons
 }
 
 // ------------------------------------------------------------------------------------------------
+// render_occ_kernel: the eval render of the occupancy-grid sampler (nerf_renderer.py:145-197) in ONE launch.  Tiles, tile
+// order, weight staging and eval_fields are render_march_kernel's; the samples of a ray are not a fixed lattice but the
+// intervals its grid walk emits (occ_walk.cuh), produced one per tile iteration by the thread that owns the ray.  A ray
+// stops at its first interval whose exclusive transmittance is below early_stop_eps (nerfacc's
+// render_visibility_from_density with alpha_thre = 0: T never increases, so no later interval could pass), i.e. only
+// the intervals that contribute are evaluated, and nothing per sample leaves the SM.  The tile iterates until its last
+// ray has stopped; rows without an interval enter eval_fields masked out.
+struct OccRenderArgs {
+    OccGrid   grid;
+    float     early_stop_eps;
+    uint32_t* n_samples;        // [R] intervals composited per ray, or null
+};
+
+template <bool PANO, bool SIMT, int NDENSE>
+__global__ void __launch_bounds__(TILE, 4) render_occ_kernel(const __grid_constant__ RenderArgs a, const __grid_constant__ OccRenderArgs g)
+{
+    extern __shared__ __align__(128) uint8_t smem[];
+    uint8_t* sA   = smem + RS_A;
+    uint8_t* sW1g = smem + RS_W1G;
+    uint8_t* sW1a = smem + RS_W1A;
+    uint8_t* sW2a = smem + RS_W2A;
+    float*   sWoutG = reinterpret_cast<float*>(smem + RS_WOUT);
+    float*   sWoutA = sWoutG + HID;
+    uint64_t* bar = reinterpret_cast<uint64_t*>(smem + RS_BAR);
+    uint32_t* tmem_slot = reinterpret_cast<uint32_t*>(smem + RS_BAR + 8);
+
+    const int tid = threadIdx.x, warp = tid >> 5;
+    const RenderSmem sm = {sA, sA, sA + A32_BYTES, sW1g, sW1a, sW2a, sWoutG, sWoutA, bar, nullptr};
+
+    stage_weights_bulk(smem, tid);                   // W1 density | W1 colour | W2 colour operand images, one UBLKCP
+    uint32_t tmem_base = 0;
+    if (!SIMT) {
+        if (tid == 0) { mbar_init(bar, 1); fence_mbar_init(); }
+        __syncwarp();
+        if (warp == 0) tmem_alloc<128>(tmem_slot);
+        fence_proxy_async();
+        tc_fence_before();
+        __syncthreads();
+        tc_fence_after();
+        tmem_base = *tmem_slot;
+    } else {
+        __syncthreads();
+    }
+    const uint32_t tmem_row = tmem_base + ((uint32_t)(warp * 32) << 16);
+    uint32_t parity = 0;
+
+    const float rext0 = __frcp_rn(a.aabb_ext[0]), rext1 = __frcp_rn(a.aabb_ext[1]), rext2 = __frcp_rn(a.aabb_ext[2]);
+    const bool patch = PANO || a.W > 0;
+    const int rows = patch ? (int)(a.R / (uint64_t)a.W) : 0;
+    const uint32_t tiles_x = patch ? (uint32_t)((a.W + PATCH_W - 1) / PATCH_W) : 0u;
+    const uint64_t n_tiles = patch ? (uint64_t)tiles_x * (uint64_t)((rows + PATCH_H - 1) / PATCH_H) : (a.R + TILE - 1) / TILE;
+
+    for (uint64_t work = blockIdx.x; work < n_tiles; work += gridDim.x) {
+        const uint64_t tile = (patch && a.tile_mul > 1u) ? (work * a.tile_mul) % n_tiles : work;
+        uint64_t ray; bool valid;
+        float o[3] = {0.f, 0.f, 0.f}, d[3] = {1.f, 0.f, 0.f};
+        march_tile_ray<PANO>(a, tile, patch, tiles_x, rows, TILE, tid, ray, valid, o[0], o[1], o[2], d[0], d[1], d[2]);
+        OccWalk walk = {0.f, 0.f, 0u, 0u};
+        if (valid) occ_walk_begin(g.grid, o, d, walk);
+
+        bool live = valid;
+        uint32_t n = 0;
+        float sum_sd = 0.f;                                   // exclusive running sum of sigma*dt
+        float acc_w = 0.f, acc_d = 0.f, acc_r = 0.f, acc_g = 0.f, acc_b = 0.f;
+#pragma unroll 1
+        for (;;) {
+            // the next interval of my ray, unless the ray is exhausted or its transmittance fell below the cut
+            float ts = 0.f, te = 0.f;
+            const float T = expf(-sum_sd);
+            live = live && T >= g.early_stop_eps && occ_walk_next(g.grid, o, d, walk, ts, te);
+            // also orders the previous iteration's reads of the feature / hidden tiles before this one's writes
+            if (!__syncthreads_or(live)) break;
+            const float tsum = __fadd_rn(ts, te);
+            const float px = __fadd_rn(o[0], __fmul_rn(d[0], tsum) * 0.5f);
+            const float py = __fadd_rn(o[1], __fmul_rn(d[1], tsum) * 0.5f);
+            const float pz = __fadd_rn(o[2], __fmul_rn(d[2], tsum) * 0.5f);
+            const float x = div_uniform(__fsub_rn(px, a.aabb_min[0]), a.aabb_ext[0], rext0, a.div_generic != 0u);
+            const float y = div_uniform(__fsub_rn(py, a.aabb_min[1]), a.aabb_ext[1], rext1, a.div_generic != 0u);
+            const float z = div_uniform(__fsub_rn(pz, a.aabb_min[2]), a.aabb_ext[2], rext2, a.div_generic != 0u);
+            const bool selector = live && x > 0.f && x < 1.f && y > 0.f && y < 1.f && z > 0.f && z < 1.f;
+
+            float sigma, cr, cg, cb;
+            eval_fields<SIMT, NDENSE>(a, sm, x, y, z, selector, tmem_base, tmem_row, parity, tid, sigma, cr, cg, cb);
+
+            if (live) {                                       // render_march_kernel's composite, same operations in the same order
+                const float sd = sigma * __fsub_rn(te, ts);
+                const float w = T * (1.f - expf(-sd));
+                sum_sd += sd;
+                acc_w += w; acc_d = fmaf(w, tsum * 0.5f, acc_d);
+                acc_r = fmaf(w, cr, acc_r); acc_g = fmaf(w, cg, acc_g); acc_b = fmaf(w, cb, acc_b);
+                ++n;
+            }
+        }
+
+        if (valid) {                                          // eval background rule, nerf_renderer.py:195-197
+            const float one_m = 1.f - acc_w;
+            a.rgb[3 * ray] = acc_r + 0.5f * one_m; a.rgb[3 * ray + 1] = acc_g + 0.5f * one_m; a.rgb[3 * ray + 2] = acc_b + 0.5f * one_m;
+            a.distance[ray] = acc_d + 5.f * one_m;
+            if (a.opacity) a.opacity[ray] = acc_w;
+            if (g.n_samples) g.n_samples[ray] = n;
+        }
+    }
+
+    if (!SIMT) {
+        tc_fence_before();
+        __syncthreads();
+        if (warp == 0) tmem_dealloc<128>(tmem_base);
+    }
+}
+
+// ------------------------------------------------------------------------------------------------
 // packed_fields_kernel: both fields at PACKED samples (the output of the occupancy sampler), thread = sample,
 // a tile = 128 CONSECUTIVE packed samples.  Consecutive samples of a ray are 5e-4 apart (nerf_renderer.py:151):
 // a warp's 32 lanes sit in one cell of every level up to resolution ~1000, the best gather locality there is.
@@ -861,49 +1019,65 @@ static void set_div_mode(RenderArgs& a)
 
 static uint32_t gcd_u32(uint32_t a, uint32_t b) { while (b) { uint32_t t = a % b; a = b; b = t; } return a; }
 
+// Table, weights, field box, flags and outputs of a render launch: everything but the sampler.  No CUDA call.
+static int fill_render_args(const perf_render_args* args, RenderArgs& a, PackedLayout& pl)
+{
+    PERF_CHECK_ARG((uintptr_t)args->d_packed_table % 16 == 0 && (uintptr_t)args->d_geo_mlp_half % 16 == 0 && (uintptr_t)args->d_app_mlp_half % 16 == 0, "misaligned table / weights");
+    uint64_t n_entries = 0;
+    int rc = build_level_table(&args->grid, &a.lt, &n_entries); if (rc) return rc;
+    PERF_CHECK_SUP(args->grid.n_levels == 16, "fused renderer needs n_levels == 16 (got %u)", args->grid.n_levels);
+    a.table = (const uint2*)args->d_packed_table;
+    pl = packed_layout(a.lt, n_entries);
+    for (uint32_t l = 0; l < pl.n_cell_levels; ++l) a.cells[l] = reinterpret_cast<const uint4*>(a.table + pl.cell_start[l]);
+    a.geo_w = (const __half*)args->d_geo_mlp_half; a.app_w = (const __half*)args->d_app_mlp_half;
+    for (int i = 0; i < 3; ++i) { a.aabb_min[i] = args->aabb[i]; a.aabb_ext[i] = args->aabb[3 + i] - args->aabb[i]; }
+    set_div_mode(a);
+    a.training = (args->flags & PERF_FLAG_TRAINING) ? 1u : 0u;
+    a.jitter = args->d_jitter; a.bg_noise = args->d_bg_noise;
+    a.rgb = args->d_rgb; a.distance = args->d_distance; a.opacity = args->d_opacity;
+    return PERF_OK;
+}
+
+#ifndef PERF_TILE_SCATTER
+#define PERF_TILE_SCATTER 1
+#endif
+// Persistent grid of a render launch (4 CTAs per SM, at most one per work tile); image-shaped work (`image`) also gets
+// its scattered tile order in a.tile_mul
+static unsigned schedule_tiles(RenderArgs& a, uint64_t n_work, bool image)
+{
+    const unsigned grid = (unsigned)(n_work < (uint64_t)num_sms() * 4 ? n_work : (uint64_t)num_sms() * 4);
+    a.tile_mul = 0;
+    if (PERF_TILE_SCATTER && image && n_work > grid && n_work < (1ull << 31)) {
+        // golden-ratio stride, made coprime with the tile count: consecutive work items land far apart, evenly spread
+        uint32_t m = (uint32_t)((double)n_work * 0.6180339887498949) | 1u;
+        while (m > 1u && gcd_u32(m, (uint32_t)n_work) != 1u) m += 2u;
+        a.tile_mul = m % (uint32_t)n_work;
+    }
+    return grid;
+}
+
 static int launch_render(const perf_render_args* args, RenderArgs& a, bool pano, cudaStream_t stream, int save = 0)
 {
     PERF_CHECK_ARG(args->d_packed_table && args->d_geo_mlp_half && args->d_app_mlp_half, "NULL table / weights");
     PERF_CHECK_ARG(args->d_rgb && args->d_distance, "NULL output");
     PERF_CHECK_ARG(args->n_samples >= 1 && args->n_samples <= 4096, "n_samples=%u not in [1,4096]", args->n_samples);
     PERF_CHECK_ARG(args->far > args->near, "far <= near");
-    PERF_CHECK_ARG((uintptr_t)args->d_packed_table % 16 == 0 && (uintptr_t)args->d_geo_mlp_half % 16 == 0 && (uintptr_t)args->d_app_mlp_half % 16 == 0, "misaligned table / weights");
-    uint64_t n_entries = 0;
-    int rc = build_level_table(&args->grid, &a.lt, &n_entries); if (rc) return rc;
-    PERF_CHECK_SUP(args->grid.n_levels == 16, "fused renderer needs n_levels == 16 (got %u)", args->grid.n_levels);
-    a.table = (const uint2*)args->d_packed_table;
-    const PackedLayout pl = packed_layout(a.lt, n_entries);
-    for (uint32_t l = 0; l < pl.n_cell_levels; ++l) a.cells[l] = reinterpret_cast<const uint4*>(a.table + pl.cell_start[l]);
-    a.geo_w = (const __half*)args->d_geo_mlp_half; a.app_w = (const __half*)args->d_app_mlp_half;
-    for (int i = 0; i < 3; ++i) { a.aabb_min[i] = args->aabb[i]; a.aabb_ext[i] = args->aabb[3 + i] - args->aabb[i]; }
+    PackedLayout pl;
+    int rc = fill_render_args(args, a, pl); if (rc) return rc;
     a.S = args->n_samples; a.near = args->near; a.far = args->far;
-    set_div_mode(a);
-    a.training = (args->flags & PERF_FLAG_TRAINING) ? 1u : 0u;
-    a.jitter = args->d_jitter; a.bg_noise = args->d_bg_noise;
-    a.rgb = args->d_rgb; a.distance = args->d_distance; a.opacity = args->d_opacity;
     const uint32_t g = gcd_u32(a.S, TILE);
     a.rays_per_unit = TILE / g; a.tiles_per_unit = a.S / g;       // unit = lcm(S,128) samples
     if (a.R == 0) return PERF_OK;
     const bool simt = (args->flags & PERF_FLAG_SIMT_MLP) != 0;
     const bool scan = (args->flags & PERF_FLAG_SCAN_KERNEL) != 0;
     uint64_t n_work;
-#ifndef PERF_TILE_SCATTER
-#define PERF_TILE_SCATTER 1
-#endif
     if (scan) n_work = (a.R + a.rays_per_unit - 1) / a.rays_per_unit;
     else if (pano || a.W > 0) n_work = (uint64_t)((a.W + PATCH_W - 1) / PATCH_W) * (uint64_t)(((int)(a.R / (uint64_t)a.W) + PATCH_H - 1) / PATCH_H);
     else {
         const uint32_t rpt = TILE / (a.seg ? a.seg : 1u);
         n_work = (a.R + rpt - 1) / rpt;
     }
-    const unsigned grid = (unsigned)(n_work < (uint64_t)num_sms() * 4 ? n_work : (uint64_t)num_sms() * 4);
-    a.tile_mul = 0;
-    if (PERF_TILE_SCATTER && !scan && (pano || a.W > 0) && n_work > grid && n_work < (1ull << 31)) {
-        // golden-ratio stride, made coprime with the tile count: consecutive work items land far apart, evenly spread
-        uint32_t m = (uint32_t)((double)n_work * 0.6180339887498949) | 1u;
-        while (m > 1u && gcd_u32(m, (uint32_t)n_work) != 1u) m += 2u;
-        a.tile_mul = m % (uint32_t)n_work;
-    }
+    const unsigned grid = schedule_tiles(a, n_work, !scan && (pano || a.W > 0));
     rc = prepare_weights(a, stream); if (rc) return rc;     // constant-bank output weights + operand images (c_wout, g_wimg)
 #define PERF_RENDER_LAUNCH(...) do { \
         auto k = __VA_ARGS__; \
@@ -933,6 +1107,54 @@ static int launch_render(const perf_render_args* args, RenderArgs& a, bool pano,
         if (pano) PERF_RENDER_LAUNCH(render_march_kernel<true, false, -1>); else PERF_RENDER_LAUNCH(render_march_kernel<false, false, -1>);
     }
 #undef PERF_RENDER_LAUNCH
+    PERF_LAUNCH_CHECK();
+    return PERF_OK;
+}
+
+// render_occ_kernel: every argument is checked before the first CUDA call
+static int launch_render_occ(const perf_render_args* args, const perf_occ_render_args* occ, RenderArgs& a, bool pano, cudaStream_t stream)
+{
+    PERF_CHECK_ARG(args->d_packed_table && args->d_geo_mlp_half && args->d_app_mlp_half, "NULL table / weights");
+    PERF_CHECK_ARG(args->d_rgb && args->d_distance, "NULL output");
+    PERF_CHECK_SUP((args->flags & (PERF_FLAG_TRAINING | PERF_FLAG_SCAN_KERNEL | PERF_FLAG_L0_SMEM)) == 0,
+                   "occupancy-grid rendering is eval mode on the ray-marching kernel (no TRAINING / SCAN_KERNEL / L0_SMEM flag)");
+    PERF_CHECK_ARG(occ->d_binaries, "NULL occupancy grid");
+    PERF_CHECK_ARG(occ->res[0] > 0 && occ->res[1] > 0 && occ->res[2] > 0, "occupancy grid resolution %d x %d x %d", occ->res[0], occ->res[1], occ->res[2]);
+    PERF_CHECK_ARG(occ->aabb[3] > occ->aabb[0] && occ->aabb[4] > occ->aabb[1] && occ->aabb[5] > occ->aabb[2], "empty occupancy grid box");
+    PERF_CHECK_ARG(occ->step > 0.f && occ->far > occ->near, "bad occupancy lattice near=%g far=%g step=%g", occ->near, occ->far, occ->step);
+    PERF_CHECK_ARG(occ->early_stop_eps >= 0.f && occ->early_stop_eps < 1.f, "early_stop_eps=%g not in [0,1)", occ->early_stop_eps);
+    PackedLayout pl;
+    int rc = fill_render_args(args, a, pl); if (rc) return rc;
+    OccRenderArgs g; memset(&g, 0, sizeof(g));
+    g.grid.binaries = occ->d_binaries;
+    for (int i = 0; i < 3; ++i) {
+        g.grid.res[i] = occ->res[i];
+        g.grid.amin[i] = occ->aabb[i]; g.grid.amax[i] = occ->aabb[3 + i]; g.grid.aext[i] = occ->aabb[3 + i] - occ->aabb[i];
+    }
+    g.grid.near = occ->near; g.grid.far = occ->far; g.grid.step = occ->step;
+    g.early_stop_eps = occ->early_stop_eps; g.n_samples = occ->d_n_samples;
+    if (a.R == 0) return PERF_OK;
+    const bool image = pano || a.W > 0;
+    const uint64_t n_work = image ? (uint64_t)((a.W + PATCH_W - 1) / PATCH_W) * (uint64_t)(((int)(a.R / (uint64_t)a.W) + PATCH_H - 1) / PATCH_H)
+                                  : (a.R + TILE - 1) / TILE;
+    const unsigned grid = schedule_tiles(a, n_work, image);
+    rc = prepare_weights(a, stream); if (rc) return rc;
+#define PERF_OCC_LAUNCH(...) do { \
+        auto k = __VA_ARGS__; \
+        static thread_local int attr_dev = -1; int dev_ = 0; PERF_CUDA(cudaGetDevice(&dev_)); \
+        if (attr_dev != dev_) { PERF_CUDA(cudaFuncSetAttribute(k, cudaFuncAttributeMaxDynamicSharedMemorySize, RS_LAUNCH)); \
+            attr_dev = dev_; } \
+        k<<<grid, TILE, RS_LAUNCH, stream>>>(a, g); } while (0)
+    const bool simt = (args->flags & PERF_FLAG_SIMT_MLP) != 0;
+    const bool fast = fast_addressing_ok(a.lt, 4) && pl.n_cell_levels == 4 && (args->flags & PERF_FLAG_GENERIC_ADDR) == 0;
+    if (pano) {
+        if (simt) { if (fast) PERF_OCC_LAUNCH(render_occ_kernel<true, true, 4>);  else PERF_OCC_LAUNCH(render_occ_kernel<true, true, -1>); }
+        else      { if (fast) PERF_OCC_LAUNCH(render_occ_kernel<true, false, 4>); else PERF_OCC_LAUNCH(render_occ_kernel<true, false, -1>); }
+    } else {
+        if (simt) { if (fast) PERF_OCC_LAUNCH(render_occ_kernel<false, true, 4>);  else PERF_OCC_LAUNCH(render_occ_kernel<false, true, -1>); }
+        else      { if (fast) PERF_OCC_LAUNCH(render_occ_kernel<false, false, 4>); else PERF_OCC_LAUNCH(render_occ_kernel<false, false, -1>); }
+    }
+#undef PERF_OCC_LAUNCH
     PERF_LAUNCH_CHECK();
     return PERF_OK;
 }
@@ -1049,6 +1271,30 @@ int perf_render_pano(const perf_render_args* args, const float* h_pose, int H, i
     for (int r = 0; r < 3; ++r) { for (int c = 0; c < 3; ++c) a.pose_r[3 * r + c] = h_pose[4 * r + c]; a.pose_t[r] = h_pose[4 * r + 3]; }
     a.H = H; a.W = W; a.row0 = row0; a.R = (uint64_t)rows * W;
     return launch_render(args, a, true, (cudaStream_t)stream);
+}
+
+int perf_render_rays_occ(const perf_render_args* args, const perf_occ_render_args* occ, const float* d_rays_o, const float* d_rays_d,
+                         uint64_t R, void* stream)
+{
+    PERF_CHECK_ARG(args && occ && d_rays_o && d_rays_d, "NULL pointer");
+    RenderArgs a; memset(&a, 0, sizeof(a));
+    a.rays_o = d_rays_o; a.rays_d = d_rays_d; a.R = R;
+    if (args->image_width > 0) {
+        PERF_CHECK_ARG(R % args->image_width == 0, "image_width=%u does not divide the %llu rays", args->image_width, (unsigned long long)R);
+        a.W = (int)args->image_width;
+    }
+    return launch_render_occ(args, occ, a, false, (cudaStream_t)stream);
+}
+
+int perf_render_pano_occ(const perf_render_args* args, const perf_occ_render_args* occ, const float* h_pose, int H, int W, int row0, int rows,
+                         void* stream)
+{
+    PERF_CHECK_ARG(args && occ && h_pose, "NULL pointer");
+    PERF_CHECK_ARG(H > 0 && W > 0 && row0 >= 0 && rows >= 0 && row0 + rows <= H, "bad panorama window H=%d W=%d row0=%d rows=%d", H, W, row0, rows);
+    RenderArgs a; memset(&a, 0, sizeof(a));
+    for (int r = 0; r < 3; ++r) { for (int c = 0; c < 3; ++c) a.pose_r[3 * r + c] = h_pose[4 * r + c]; a.pose_t[r] = h_pose[4 * r + 3]; }
+    a.H = H; a.W = W; a.row0 = row0; a.R = (uint64_t)rows * W;
+    return launch_render_occ(args, occ, a, true, (cudaStream_t)stream);
 }
 
 #pragma GCC visibility pop

@@ -598,6 +598,67 @@ def render_pano(packed_table, geo_mlp_half, app_mlp_half, pose, H: int, W: int, 
     return rgb, dist, op
 
 
+def _occ_render_args(binaries: torch.Tensor, grid_aabb, near: float, far: float, step: float, early_stop_eps: float,
+                     n_samples: Optional[torch.Tensor]) -> "_lib.OccRenderArgs":
+    if not isinstance(binaries, torch.Tensor) or not binaries.is_cuda or binaries.dim() != 3:
+        raise RuntimeError("perf_b200: `binaries` must be a CUDA bool / uint8 tensor [rx, ry, rz]")
+    if not binaries.is_contiguous():
+        raise ValueError("perf_b200: `binaries` must be contiguous")
+    bins = binaries.view(torch.uint8) if binaries.dtype == torch.bool else _chk(binaries, torch.uint8, "binaries")
+    g = _lib.OccRenderArgs()
+    g.d_binaries = bins.data_ptr()
+    g.res = (C.c_int * 3)(*[int(v) for v in binaries.shape])
+    g.aabb = (C.c_float * 6)(*[float(v) for v in grid_aabb])
+    g.near, g.far, g.step, g.early_stop_eps = float(near), float(far), float(step), float(early_stop_eps)
+    g.d_n_samples = None if n_samples is None else n_samples.data_ptr()
+    return g
+
+
+def render_rays_occ(packed_table, geo_mlp_half, app_mlp_half, rays_o, rays_d, binaries, grid_aabb, near=0.0, far=1.5, step=5e-4,
+                    early_stop_eps=1e-4, aabb=(-1., -1., -1., 1., 1., 1.), grid: GridConfig = PERF_GRID, simt=False,
+                    image_width: int = 0, want_n_samples: bool = False, kernel: str = "march"):
+    """One-launch eval render of explicit rays [R,3] with the occupancy-grid sampler inside the kernel (grid walk, both
+    fields, composite with the ``early_stop_eps`` transmittance cut) -> (rgb [R,3], distance [R,1], opacity [R,1]) and, with
+    ``want_n_samples``, the intervals composited per ray [R] int32 as a fourth element.  ``binaries`` [rx,ry,rz] and
+    ``grid_aabb`` are the estimator's grid and roi; ``aabb`` is the field's box.  No host read, no allocation besides
+    the outputs (capturable into a CUDA graph)."""
+    rays_o, rays_d = _chk(rays_o, torch.float32, "rays_o"), _chk(rays_d, torch.float32, "rays_d")
+    R, dev = rays_o.shape[0], rays_o.device
+    rgb = torch.empty(R, 3, dtype=torch.float32, device=dev)
+    dist = torch.empty(R, 1, dtype=torch.float32, device=dev)
+    op = torch.empty(R, 1, dtype=torch.float32, device=dev)
+    n = torch.empty(R, dtype=torch.int32, device=dev) if want_n_samples else None
+    if R == 0:
+        return (rgb, dist, op, n) if want_n_samples else (rgb, dist, op)
+    a = _render_args(packed_table, geo_mlp_half, app_mlp_half, aabb, 1, 0.0, 1.0, False, simt, None, None, rgb, dist, op, grid, kernel)
+    a.image_width = int(image_width) if image_width and R % int(image_width) == 0 else 0
+    g = _occ_render_args(binaries, grid_aabb, near, far, step, early_stop_eps, n)
+    with torch.cuda.device(dev):
+        _call(_L().perf_render_rays_occ, C.byref(a), C.byref(g), _p(rays_o), _p(rays_d), R, _stream())
+    return (rgb, dist, op, n) if want_n_samples else (rgb, dist, op)
+
+
+def render_pano_occ(packed_table, geo_mlp_half, app_mlp_half, pose, H: int, W: int, binaries, grid_aabb, near=0.0, far=1.5, step=5e-4,
+                    early_stop_eps=1e-4, row0: int = 0, rows: Optional[int] = None, aabb=(-1., -1., -1., 1., 1., 1.),
+                    grid: GridConfig = PERF_GRID, simt=False, out=None, want_n_samples: bool = False, kernel: str = "march"):
+    """:func:`render_rays_occ` for rows [row0,row0+rows) of an HxW equirect panorama, ray generation fused in.
+    Returns (rgb [rows,W,3], distance [rows,W,1], opacity [rows,W,1]) (+ n_samples [rows,W] int32)."""
+    rows = H - row0 if rows is None else rows
+    dev = packed_table.device
+    if out is None:
+        rgb = torch.empty(rows, W, 3, dtype=torch.float32, device=dev)
+        dist = torch.empty(rows, W, 1, dtype=torch.float32, device=dev)
+        op = torch.empty(rows, W, 1, dtype=torch.float32, device=dev)
+    else:
+        rgb, dist, op = out
+    n = torch.empty(rows, W, dtype=torch.int32, device=dev) if want_n_samples else None
+    a = _render_args(packed_table, geo_mlp_half, app_mlp_half, aabb, 1, 0.0, 1.0, False, simt, None, None, rgb, dist, op, grid, kernel)
+    g = _occ_render_args(binaries, grid_aabb, near, far, step, early_stop_eps, n)
+    with torch.cuda.device(dev):
+        _call(_L().perf_render_pano_occ, C.byref(a), C.byref(g), _pose_array(pose), H, W, row0, rows, _stream())
+    return (rgb, dist, op, n) if want_n_samples else (rgb, dist, op)
+
+
 # ------------------------------------------------------------------ fused training step
 class FusedTrainContext:
     """Everything one fused training step needs besides the rays: the fp16 shadows / gather table,

@@ -424,6 +424,11 @@ class NeRFScene:
             self.fused.set_halves(self.nerf.geo_mlp._half(), self.nerf.app_mlp._half())
             self._fused_key = key
 
+    def _sync_occupancy(self):
+        """The estimator's current grid (a view: in-place updates are seen) as the fused renderer's occupancy grid."""
+        est = self.estimator
+        self.fused.set_occupancy(est.binaries[0], est._aabb_list(), near=0.0, far=1.5, step=self.OCC_STEP, early_stop_eps=1e-4)
+
     @torch.no_grad()
     def render(self, rays: Rays, query_keys=("rgb",), sampling_requires_grad=False):
         """`nerf.py:74-99`: eval-mode render of arbitrarily shaped rays -> {key: [..., C]}."""
@@ -434,12 +439,10 @@ class NeRFScene:
         rays_o_img, rays_d_img = rays_o.float(), rays_d.float()
         rays_o, rays_d = rays_o.reshape(-1, 3).float(), rays_d.reshape(-1, 3).float()
         if self.estimator_type == "occ":
-            # nerf_renderer.py:145-197: occupancy sampling, both fields at every interval (one launch), composite with
-            # nerfacc's 1e-4 transmittance cut applied inside (identical to culling first; see csrc/packed.cu)
-            est = self.estimator
-            ri, ts, te = ops.occ_sample(est.binaries[0], est._aabb_list(), rays_o.contiguous(), rays_d.contiguous(), 0.0, 1.5,
-                                        self.OCC_STEP, None)
-            out = self.fused.render_occ(rays_o, rays_d, ops.occ_sample.last_offsets, ri, ts, te, early_stop_eps=1e-4)
+            # nerf_renderer.py:145-197 in one launch: each ray walks the occupancy grid, evaluates both fields at the
+            # intervals it emits and stops at nerfacc's 1e-4 transmittance cut (csrc/render.cu::render_occ_kernel)
+            self._sync_occupancy()
+            out = self.fused.render_rays_occ(rays_o_img if image else rays_o, rays_d_img if image else rays_d)
         else:
             out = self.fused.render_rays(rays_o_img if image else rays_o, rays_d_img if image else rays_d, self.estimator.n_samples)
         return {k: out[k].reshape(pre_shape + [-1]) for k in query_keys}
@@ -449,10 +452,8 @@ class NeRFScene:
         """render_dense inner loop (`core_exp_runner.py:229-238`) with ray generation fused in."""
         self._sync_fused()
         if self.estimator_type == "occ":
-            rows = height - row0 if rows is None else rows
-            o, d = ops.raygen_pano(pose, height, width, row0, rows, device=self.device)
-            out = self.render(Rays(o, d), ["rgb", "distance", "opacities"])
-            return {**out, "is_valid": True}
+            self._sync_occupancy()
+            return self.fused.render_pano_occ(pose, height, width, row0=row0, rows=rows)
         return self.fused.render_pano(pose, height, width, self.estimator.n_samples, row0=row0, rows=rows)
 
     @torch.no_grad()
